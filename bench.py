@@ -42,6 +42,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ for the modules imported from it
 
 METRIC = "scan_to_map_lidar_frames_per_sec"
 KEYFRAME_EVERY = 10
@@ -52,6 +53,7 @@ CONFIGS = {
     "C5": dict(lidars=8, rings=128, horizon=2048, map_points=10_000_000, gn_iters=10, gf_method=3, gf_ratio=0.8, calib=False),
 }
 DEFAULT_CONFIG = {1: "C2", 2: "C3", 4: "C4", 8: "C5"}
+SOLVE_STATS = ("ran", "n_surf", "n_corner", "lm_iterations", "degenerate", "termination", "final_cost", "eig", "H", "n_surf_in", "n_corner_in")
 KNN_BYTES_PER_FEATURE = 16 + 5 * 16 + 5 * 4   # k_match_knn: query float4 + 5 neighbour float4 + 5 neighbour positions
 MAP_BYTES_PER_POINT = 40                     # map build: 16 read + 16 sorted write + 8 key/rank (SURVEY.md §8d)
 
@@ -467,6 +469,17 @@ def gpu_measure(m, syn, torch, dist, cfg_name, cfg, args, rank, local_rank, worl
     return res
 
 
+def dump_outputs(out_dir: str, R: dict, calib: bool) -> None:
+    """--dump-outputs: what the timed call returned in its last timed step (the solved pose, or pose_i and ext_cal of a calibration
+    step, and every field of the solve statistics), one float64 DIR/<name>.npy each.  The workload is seeded, so two builds run
+    with the same arguments can be compared file by file."""
+    outs = {"pose_i": R["last_pose"], "ext_cal": R["last_ext"]} if calib else {"pose": R["last_pose"]}
+    outs.update((k, R["last_stats"][k]) for k in SOLVE_STATS)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+
 def config_blurb(name, cfg, n_gpus, args, wl):
     per = max(1, cfg["lidars"] // n_gpus)
     return {"workload": f"{name}: {cfg['lidars']} LiDAR(s) x {cfg['rings']}-ring x {cfg['horizon']} sweep, {cfg['map_points']}-pt edge+surf submap (1:9), "
@@ -495,7 +508,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-lookahead", action="store_true", help="do not announce sweep k+1 while frame k runs (no overlap of extraction with the solve)")
     ap.add_argument("--no-c4", action="store_true", help="skip the extra C4-on-one-GPU measurement of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU arm (--impl ours)")
 
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ and args.impl == "ours":
         # N > 1 is one process per GPU: when not already under torchrun, relaunch this command under it
@@ -601,6 +620,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, R, cfg["calib"])
 
     wl = R["wl"]
     config = config_blurb(cfg_name, cfg, n_gpus, args, wl)

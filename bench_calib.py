@@ -126,7 +126,7 @@ def gpu_measure_calib(m, syn, torch, dist, cfg_name, cfg, args, rank, local_rank
                keyframe_ms=statistics.mean(ms_steps[0::KF]), regular_ms=(statistics.mean([x for i, x in enumerate(ms_steps) if i % KF]) if KF > 1 and steps > 1 else None),
                clocks=clocks, launches=int(ctx.launch_count() - launches0), exchange=exchange, exchange_timeouts=0,
                features_per_step=float(sum(cs0[k].shape[0] for k in ("surf_ref", "corner_ref", "surf_cal", "corner_cal"))),
-               t_max=t_max, value=L * steps / t_max, k_last=(steps - 1) % len(cases), last_pose=last[0], last_stats=last[2],
+               t_max=t_max, value=L * steps / t_max, k_last=(steps - 1) % len(cases), last_pose=last[0], last_ext=last[1], last_stats=last[2],
                wl={"map_info": map_info, "cases": cases},
                e2e={"value": L * steps / t_e2e, "unit": "frames/s", "h2d_bytes_per_step": int(feat_bytes + map_bytes * n_kf / steps), "d2h_bytes_per_step": 2000,
                     "steps": steps, "h2d_detail": {"features_every_step": feat_bytes, "local_maps_on_keyframe_steps": map_bytes, "keyframe_steps": n_kf}})

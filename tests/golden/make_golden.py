@@ -34,9 +34,19 @@ def small_case():
     return surf_map, corner_map, cloud, ss, se, init
 
 
+def knn_uniform():
+    """knn_nanoflann_uniform.npz: the reference kd-tree's answers on test_oracle_cpu.knn_uniform_case() (the map is re-made from its seed)."""
+    from test_oracle_cpu import knn_uniform_case
+    m, q = knn_uniform_case()
+    out = {"query": q}
+    for k in (1, 5, 10):
+        out[f"idx{k}"], out[f"sqd{k}"] = orc.ref_knn(m, q, k)
+    np.savez_compressed(os.path.join(HERE, "knn_nanoflann_uniform.npz"), **out)
+
+
 def main():
     # ---- reference nanoflann
-    assert orc.ref_lib() is not None, "oracle/_ref/libref_knn.so missing: run `make -C oracle ref` where /root/reference exists"
+    assert orc.ref_lib() is not None, "oracle/_ref/libref_knn.so missing: run `make -C oracle ref` where the reference sources are"
     rng = np.random.default_rng(2024)
     m = np.concatenate([rng.uniform(-8, 8, (6000, 3)), np.zeros((6000, 1))], 1).astype(np.float32)
     q = np.concatenate([rng.uniform(-8.5, 8.5, (300, 3)), np.zeros((300, 1))], 1).astype(np.float32)
@@ -45,6 +55,7 @@ def main():
         idx, sqd = orc.ref_knn(m, q, k)
         out[f"idx{k}"], out[f"sqd{k}"] = idx, sqd
     np.savez_compressed(os.path.join(HERE, "knn_nanoflann.npz"), **out)
+    knn_uniform()
 
     # ---- oracle regression vectors
     surf_map, corner_map, cloud, ss, se, init = small_case()
@@ -66,7 +77,7 @@ def main():
     import synthetic as syn
     surf_f, corner_f = syn.keyframe_map_features(syn.make_scene(), orc.extract_cloud, orc.voxel_grid, use_cache=False)
     np.savez_compressed(os.path.join(HERE, "submap_keyframes_filtered.npz"), surf=surf_f, corner=corner_f, tag=f"{syn.SEED}_30_64x2048")
-    for name in ("knn_nanoflann.npz", "oracle_small.npz", "submap_keyframes_filtered.npz"):
+    for name in ("knn_nanoflann.npz", "knn_nanoflann_uniform.npz", "oracle_small.npz", "submap_keyframes_filtered.npz"):
         print(name, os.path.getsize(os.path.join(HERE, name)), "bytes")
 
 

@@ -985,3 +985,28 @@ def test_golden_oracle_vectors_on_gpu(ctx):
         ctx.set_params(max_outer=2, max_inner=30)
     dt, dr = syn.pose_err(pose, g["pose"])
     assert dt <= POSE_TOL_T and dr <= POSE_TOL_R and st["n_surf"] == int(g["n_surf"]) and st["n_corner"] == int(g["n_corner"])
+
+
+def test_bench_dump_outputs_repeat(tmp_path):
+    """bench.py --dump-outputs: two runs with the same arguments write the same float64 arrays of the last timed step (seeded
+    inputs, deterministic path), far below 64 MB, and the result line reports the requested number of timed steps."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    bench = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py")
+    runs = []
+    for name in ("a", "b"):
+        d = tmp_path / name
+        out = subprocess.run([sys.executable, bench, "--steps", "3", "--warmup", "0", "--no-cpu-baseline", "--no-c4", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
+        assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 3
+        runs.append({f: np.load(d / f) for f in sorted(os.listdir(d))})
+    a, b = runs
+    assert sorted(a) == sorted(b) and "pose.npy" in a and "H.npy" in a
+    for f in a:
+        assert a[f].dtype == np.float64 and np.array_equal(a[f], b[f]), f
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    assert a["ran.npy"] == 1 and a["n_surf.npy"] > 1000

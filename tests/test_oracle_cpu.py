@@ -1,5 +1,5 @@
 """CPU tests: the oracle against analytic known answers, brute force and the reference's own kd-tree
-(oracle/_ref, built from /root/reference/mloam_loop/.../nanoflann.hpp).  The reference ships no golden
+(its answers stored under tests/golden/ by make_golden.py).  The reference ships no golden
 vectors for this path (SURVEY.md §4), so known answers are derived analytically with the conventions of the
 reference's check() printers (eps 1e-6, right-multiplied deltaQ; lidar_map_factor.hpp:72-120)."""
 import math
@@ -17,18 +17,25 @@ def rand_pose(rng):
     return syn.pose7(rng.normal(size=3) * 3, q)
 
 
-def test_knn_tree_vs_brute_and_reference_nanoflann():
+def knn_uniform_case():
+    """Seeded 20k-point map and 500 queries; tests/golden/knn_nanoflann_uniform.npz holds the reference kd-tree's answers on them."""
     rng = np.random.default_rng(1)
     m = np.concatenate([rng.uniform(-20, 20, (20000, 3)), np.zeros((20000, 1))], 1).astype(np.float32)
     q = np.concatenate([rng.uniform(-20, 20, (500, 3)), np.zeros((500, 1))], 1).astype(np.float32)
+    return m, q
+
+
+def test_knn_tree_vs_brute_and_reference_nanoflann():
+    m, q = knn_uniform_case()
+    g = np.load(os.path.join(GOLDEN, "knn_nanoflann_uniform.npz"))
+    assert np.array_equal(q, g["query"]), "the seeded inputs no longer match the stored reference answers"
     for k in (1, 5, 10):
         i_t, d_t = orc.knn(m, q, k)
         i_b, d_b = orc.knn(m, q, k, brute=True)
         assert np.array_equal(i_t, i_b) and np.array_equal(d_t, d_b)
-        if orc.ref_lib() is not None:  # the reference's vendored nanoflann, compiled where it lies
-            i_r, d_r = orc.ref_knn(m, q, k)
-            assert np.array_equal(d_t, d_r)
-            assert np.array_equal(i_t, i_r)
+        # the reference's vendored nanoflann on the same map and queries (stored by tests/golden/make_golden.py)
+        assert np.array_equal(d_t, g[f"sqd{k}"])
+        assert np.array_equal(i_t, g[f"idx{k}"])
 
 
 def test_knn_small_map_missing_slots():
