@@ -433,7 +433,7 @@ int mloam_normal_equations(mloam_ctx_t *h, int n, const unsigned char *h_types, 
   int rc = upload_pose(c, pose7, &d_pose);
   if (rc) return rc;
   MLOAM_CUDA_OK(c, c->scratch[6].reserve(sizeof(double) * 32));
-  rc = linearize_device(c, sets, 2, sqrt_info, huber_a, d_pose, 0, 0, c->scratch[6].as<double>());
+  rc = linearize_device(c, sets, 2, SolveCfg{sqrt_info, huber_a, 0.0, false}, kEvalAtPose, d_pose, c->scratch[6].as<double>());
   if (rc) return rc;
   double *ne = reinterpret_cast<double *>(c->pinned) + 64;
   MLOAM_CUDA_OK(c, cudaMemcpyAsync(ne, c->scratch[6].p, sizeof(double) * 30, cudaMemcpyDeviceToHost, c->stream));

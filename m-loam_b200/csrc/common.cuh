@@ -196,7 +196,6 @@ struct LMState {
   int n_valid[2];          // matched corner / surf features
   int max_inner;
   int pad;
-  int work[2];             // dynamic work-queue heads of the corner / surf match launches (reset by k_lm)
   int min_corr;            // a Solve with fewer matched features is skipped (lidar_tracker.cpp:64-68)
   int skipped;             // ... and this flag is raised
   long long dbg_cycles[4]; // SM cycles spent in lm_tail since k_lm_init: [0] stage-in + reduction, [1] state machine, [2] calls

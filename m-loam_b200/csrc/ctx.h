@@ -30,7 +30,8 @@ struct FitSet {
   int is_plane;
   const unsigned char *changed;  // nullable: 0 -> same neighbours as the previous iteration, valid/coeff already hold the fit
 };
-// A fit whose launch the matcher left to the first evaluation of the solve (k_linearize pass 0)
+// A fit whose launch the matcher left to the first evaluation of the solve (k_linearize pass 0): filled by
+// match_pair_device, handed by the caller to the linearize_device that begins the solve
 struct PendingFit {
   FitSet set[2];
   int K = 0;  // 0: nothing pending
@@ -230,13 +231,8 @@ struct Ctx {
   int knn_min_blocks = 4;          // k_match_knn variant: resident CTAs per SM it is compiled for (MLOAM_KNN_MB = 2 | 3 | 4)
   int use_seeds = 1;               // seed the kNN of re-association iterations > 0 with the previous neighbour lists
   int s2m_ran = 0;
-  int lm_min_corr = 0;              // lm_init_state: minimum matched features for a Solve (tracker: 10)
-  double lm_eig_thre = -1.0;        // < 0: use params.eig_thre; the tracker disables evalDegenracy with 0
   int fuse_iter = 1;               // scan2map: fit inside the first evaluation + both evaluations of an LM iteration in ONE launch
                                    // (grid barrier between them); MLOAM_FUSE_ITER=0 restores the three launches
-  PendingFit pending_fit;          // set by match_pair_device(defer_fit), consumed by the next linearize_device(lm_mode 1)
-  bool lin_two_pass = false;       // request (scan2map_enqueue) -> linearize_device clears it when it could not honour it
-  int want_eig = 1;                // k_lm mode 1: always run the 6x6 eigen-solver (1) or only when degenerate (0)
   bool lidar_merge = false;        // mloam_set_lidars was given extrinsics: features go through the rig merge (also for one LiDAR)
   int n_lidars = 1;                // LiDARs batched into one frame of this context (mloam_set_lidars)
   double lidar_ext[MLOAM_MAX_LIDARS][7];  // their sensor -> base extrinsics
@@ -251,7 +247,6 @@ struct Ctx {
   void *p2p_peer[MLOAM_P2P_MAX_RANKS] = {nullptr};
   void *p2p_view = nullptr;        // device copy of the P2PView the kernels read
   bool p2p_on = false;
-  bool p2p_collective = false;     // the solve being enqueued is the collective one (all ranks in lock-step): sum over the ranks
 };
 
 // RAII-less helper: bracket a kernel (or a few) with events when profiling is on.
@@ -281,7 +276,7 @@ int knn_device(Ctx *c, int slot, const float4 *d_q, int nq, const double *d_pose
 // type 'c' / 's'.  d_pose7 device pointer to 7 doubles.  Outputs: valid[n], coeff[n*6] float, nn[n*n_neigh] (nullable)
 // d_n (nullable): device-side feature count, n is then the launch upper bound.
 int match_from_map_device(Ctx *c, int slot, int type, const float4 *d_pts, int n, const int *d_n, const double *d_pose7,
-                          const MatchCfg &cfg, unsigned char *d_valid, float *d_coeff, int *d_nn, int *d_work = nullptr);
+                          const MatchCfg &cfg, unsigned char *d_valid, float *d_coeff, int *d_nn);
 
 // match_kernels.cu: one kNN launch + one fit launch over up to two feature sets
 struct MatchJob {
@@ -297,9 +292,10 @@ struct MatchJob {
                             // lists (Ctx::knn_pos) seed the search and unchanged lists keep their fit
 };
 // buf_base: which pair of the context's per-set buffers (knn_pos / knn_anchor / ...) the jobs use: 0 (sets 0, 1) or 2 (sets 2, 3)
-// defer_fit: skip the fit launch and leave the fit to the next linearize_device(lm_mode 1) on this context (Ctx::pending_fit)
-int match_pair_device(Ctx *c, const MatchJob *jobs, int n_jobs, const double *d_pose7, const MatchCfg &cfg, int *d_work, int buf_base = 0,
-                      bool defer_fit = false);
+// defer (nullable): when no job asks for neighbour lists, skip the fit launch and describe the fit in *defer for the
+// linearize_device that begins the solve; otherwise the fit is launched here and defer->K is 0
+int match_pair_device(Ctx *c, const MatchJob *jobs, int n_jobs, const double *d_pose7, const MatchCfg &cfg, int buf_base = 0,
+                      PendingFit *defer = nullptr);
 
 // track_kernels.cu
 int match_from_scan_device(Ctx *c, int slot, int type, const float4 *d_pts, int n, const double *d_pose7, unsigned char *d_valid,
@@ -319,12 +315,26 @@ struct FeatSet {
   const double *sinfo;         // nullable per-feature sqrt_info (with_ua: lidar_map_factor.hpp:34,41 on the point's covariance)
   const unsigned char *mask;   // nullable: only features with mask[i] != 0 enter (good-feature selection)
 };
-// Accumulate loss-corrected normal equations of both feature sets at pose *d_pose7 (or LMState x / xc when
-// use_state != 0: 1 -> x, 2 -> xc) into c->partials, then run the LM state machine step (`lm_mode`):
-//   0: none (partials only, reduced into d_out28 if non-null)   1: begin Solve   2: iterate
-int linearize_device(Ctx *c, const FeatSet *sets, int n_sets, double sqrt_info, double huber_a, const double *d_pose7,
-                     int use_state, int lm_mode, double *d_out29);
-int lm_init_state(Ctx *c, const double *pose7_host, int max_inner, double eig_thre);
+// Settings fixed for the length of one solve
+struct SolveCfg {
+  double sqrt_info;  // weight of a feature without a per-feature sqrt_info
+  double huber_a;    // HuberLoss scale
+  double eig_thre;   // evalDegenracy: directions of H with an eigenvalue below it are not updated (0: no test)
+  bool collective;   // every rank runs this solve in lock-step: the normal equations are summed over the ranks
+};
+// What linearize_device evaluates and which LM step follows (the value is lm_tail's mode)
+enum LinEval {
+  kEvalAtPose = 0,     // at d_pose7; no step (the packed normal equations go to d_out30 if non-null)
+  kEvalBegin = 1,      // at LMState::x; begins the Solve
+  kEvalCandidate = 2,  // at LMState::xc; accepts or rejects the candidate (nothing happens once the Solve is done)
+};
+// Accumulate loss-corrected normal equations of both feature sets into c->partials, then run the LM step of `eval`.
+// fit (nullable, kEvalBegin): the matcher's deferred fit, run by the evaluation at x.  two_pass: also evaluate the
+// candidate of the step in the same launch when the tail runs fused; *two_pass_done (nullable) tells whether it did.
+int linearize_device(Ctx *c, const FeatSet *sets, int n_sets, const SolveCfg &cfg, LinEval eval, const double *d_pose7 = nullptr,
+                     double *d_out30 = nullptr, const PendingFit *fit = nullptr, bool two_pass = false, bool *two_pass_done = nullptr);
+// min_corr: a Solve with fewer matched features is skipped
+int lm_init_state(Ctx *c, const double *pose7_host, int max_inner, int min_corr);
 void eig_report_host(const double *H36, double *w6);  // ascending eigenvalues of a symmetric 6x6 (host side)
 int factor_evaluate_device(Ctx *c, int kind, int n, const double *d_points, const double *d_coeffs, const double *d_sqrt_info,
                            const double *d_params, double *d_res, double *d_jac);

@@ -247,8 +247,8 @@ __global__ void __launch_bounds__(128) k_match_fit(FitSet a, FitSet b, const dou
 // ------------------------------------------------------------------------------------------------ launchers
 // Match up to two feature sets (corner against MLOAM_MAP_CORNER-like slot, surf against a surf slot) in one
 // kNN launch + one fit launch.  Sets with n == 0 are skipped.
-int match_pair_device(Ctx *c, const MatchJob *jobs, int n_jobs, const double *d_pose7, const MatchCfg &cfg, int *d_work, int buf_base, bool defer_fit) {
-  (void)d_work;
+int match_pair_device(Ctx *c, const MatchJob *jobs, int n_jobs, const double *d_pose7, const MatchCfg &cfg, int buf_base, PendingFit *defer) {
+  if (defer) defer->K = 0;
   if (n_jobs < 1 || n_jobs > 2 || (buf_base != 0 && buf_base != 2)) {
     c->err = "match: 1 or 2 jobs";
     return MLOAM_E_INVALID;
@@ -299,8 +299,8 @@ int match_pair_device(Ctx *c, const MatchJob *jobs, int n_jobs, const double *d_
     n_upper += J.n;
   }
   if (n_upper <= 0) return MLOAM_OK;
-  // heavy list of the launch: 2 lists x n_upper ints + 3 rotating counters (zeroed with the buffer; k_lm_init re-zeroes
-  // them at the start of every solve, where the rotation restarts)
+  // heavy list of the launch: 2 lists x n_upper ints + 3 rotating counters (zeroed with the buffer, and again by the
+  // non-seeded launch that starts a solve, where the rotation restarts)
   HeavyQ hq{nullptr, nullptr, nullptr, nullptr, nullptr};
   {
     DevBuf &hl = c->knn_heavy_list;
@@ -350,10 +350,9 @@ int match_pair_device(Ctx *c, const MatchJob *jobs, int n_jobs, const double *d_
 #undef MLOAM_LAUNCH_KNN
     c->launches++;
   }
-  c->pending_fit.K = 0;
-  if (defer_fit && !fs[0].nn && !fs[1].nn) {
-    c->pending_fit.set[0] = fs[0], c->pending_fit.set[1] = fs[1];
-    c->pending_fit.K = K, c->pending_fit.min_plane_dis = cfg.min_plane_dis, c->pending_fit.check_fov = cfg.check_fov;
+  if (defer && !fs[0].nn && !fs[1].nn) {
+    defer->set[0] = fs[0], defer->set[1] = fs[1];
+    defer->K = K, defer->min_plane_dis = cfg.min_plane_dis, defer->check_fov = cfg.check_fov;
   } else {
     ProfScope ps(c, "fit");
     int nb = (n_upper + 127) / 128;
@@ -367,9 +366,9 @@ int match_pair_device(Ctx *c, const MatchJob *jobs, int n_jobs, const double *d_
 }
 
 int match_from_map_device(Ctx *c, int slot, int type, const float4 *d_pts, int n, const int *d_n, const double *d_pose7,
-                          const MatchCfg &cfg, unsigned char *d_valid, float *d_coeff, int *d_nn, int *d_work) {
+                          const MatchCfg &cfg, unsigned char *d_valid, float *d_coeff, int *d_nn) {
   MatchJob j{slot, type, d_pts, n, d_n, d_valid, d_coeff, d_nn, 0};
-  return match_pair_device(c, &j, 1, d_pose7, cfg, d_work);
+  return match_pair_device(c, &j, 1, d_pose7, cfg);
 }
 
 }  // namespace mloam

@@ -470,13 +470,13 @@ extern "C" int mloam_calib_frame(mloam_ctx_t *h, const mloam_point_t *h_surf_ref
     if (n_corner_ref + n_surf_ref > 0) {
       MatchJob jobs[2] = {MatchJob{MLOAM_MAP_CORNER, 'c', sets.pts[0], ns[0], nullptr, c->feat_valid[0].as<unsigned char>(), c->feat_coeff[0].as<float>(), nullptr, 0},
                           MatchJob{MLOAM_MAP_SURF, 's', sets.pts[1], ns[1], nullptr, c->feat_valid[1].as<unsigned char>(), c->feat_coeff[1].as<float>(), nullptr, 0}};
-      rc = match_pair_device(c, jobs, 2, d_pose_a, cfg_ref, nullptr, 0);
+      rc = match_pair_device(c, jobs, 2, d_pose_a, cfg_ref, 0);
       if (rc) break;
     }
     if (n_corner_cal + n_surf_cal > 0) {
       MatchJob jobs[2] = {MatchJob{cal_corner, 'c', sets.pts[2], ns[2], nullptr, c->feat_valid[2].as<unsigned char>(), c->feat_coeff[2].as<float>(), nullptr, 0},
                           MatchJob{cal_surf, 's', sets.pts[3], ns[3], nullptr, c->feat_valid[3].as<unsigned char>(), c->feat_coeff[3].as<float>(), nullptr, 0}};
-      rc = match_pair_device(c, jobs, 2, d_pose_b, cfg_cal, nullptr, 2);
+      rc = match_pair_device(c, jobs, 2, d_pose_b, cfg_cal, 2);
       if (rc) break;
     }
     rc = calib_eval(c, sets, st, nb, partials, 0, 1);

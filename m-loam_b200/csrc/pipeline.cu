@@ -27,29 +27,27 @@ int scan2map_enqueue(Ctx *c, const ScanRef &S, const double *pose_init7) {
   if (!MS.built || !MC.built) return fail(c, MLOAM_E_STATE, "scan2map: build MLOAM_MAP_SURF and MLOAM_MAP_CORNER first");
   if (!((MS.m > 50) && (MC.m > 10))) return MLOAM_OK;  // lidar_mapper_keyframe.cpp:429 ("Map surf num is not enough")
   c->s2m_ran = 1;
-  // Collective participation: the gate above depends on the replicated maps only, so every rank takes the same branch; from here
-  // on every rank enqueues the same number of LM evaluations (max_outer x (1 + max_inner) with max_inner == 1; with max_inner > 1
-  // the done flag all ranks poll is the identical, summed state).  Per-rank solves (tracker, odometry) never set the flag.
-  struct CollectiveScope {
-    Ctx *c;
-    explicit CollectiveScope(Ctx *cc) : c(cc) { c->p2p_collective = true; }
-    ~CollectiveScope() { c->p2p_collective = false; }
-  } collective_scope(c);
+  // Collective solve: the gate above depends on the replicated maps only, so every rank takes the same branch; from here on
+  // every rank enqueues the same number of LM evaluations (max_outer x (1 + max_inner) with max_inner == 1; with max_inner > 1
+  // the done flag all ranks poll is the identical, summed state).  Per-rank solves (tracker, odometry) are not collective.
+  const SolveCfg solve{map_sqrt_info(P.cov_trace), P.huber_a, P.eig_thre, true};
   int rc = reserve_feat(c, 0, S.n_corner);
   if (rc) return rc;
   rc = reserve_feat(c, 1, S.n_surf);
   if (rc) return rc;
-  rc = lm_init_state(c, pose_init7, P.max_inner, P.eig_thre);
+  rc = lm_init_state(c, pose_init7, P.max_inner, 0);
   if (rc) return rc;
   LMState *st = c->lm_state.as<LMState>();
   const double *d_pose = st->x;  // first member
-  const double sinfo = map_sqrt_info(P.cov_trace);
   const MatchCfg cfg = match_cfg(c);
   int *h_done = reinterpret_cast<int *>(reinterpret_cast<char *>(c->pinned) + 2048);
   const int nc_use = P.point_edge_factor ? S.n_corner : 0, ns_use = P.point_plane_factor ? S.n_surf : 0;
   FeatSet sets[2] = {
       FeatSet{S.corner, c->feat_valid[0].as<unsigned char>(), c->feat_coeff[0].as<float>(), nc_use, 0, S.d_n_corner, S.sinfo_corner},
       FeatSet{S.surf, c->feat_valid[1].as<unsigned char>(), c->feat_coeff[1].as<float>(), ns_use, 1, S.d_n_surf, S.sinfo_surf}};
+  // without good-feature selection nothing reads the fit before the solve: its launch folds into the first evaluation
+  PendingFit fit;
+  PendingFit *const defer = (c->fuse_iter && P.gf_method == 0) ? &fit : nullptr;
   for (int outer = 0; outer < P.max_outer; outer++) {
     // :503-532  match corner then surf at pose_wmap_curr (wo_gf: every feature)
     {
@@ -61,9 +59,7 @@ int scan2map_enqueue(Ctx *c, const ScanRef &S, const double *pose_init7) {
                    c->feat_coeff[0].as<float>(), nullptr, seeded},
           MatchJob{MLOAM_MAP_SURF, 's', S.surf, ns_use, S.d_n_surf, c->feat_valid[1].as<unsigned char>(),
                    c->feat_coeff[1].as<float>(), nullptr, seeded}};
-      // without good-feature selection nothing reads the fit before the solve: its launch folds into the first evaluation
-      const bool defer_fit = c->fuse_iter && P.gf_method == 0;
-      rc = match_pair_device(c, jobs, 2, d_pose, cfg, &st->work[0], 0, defer_fit);
+      rc = match_pair_device(c, jobs, 2, d_pose, cfg, 0, defer);
       if (rc) return rc;
       stamp(c, "match");
     }
@@ -82,7 +78,7 @@ int scan2map_enqueue(Ctx *c, const ScanRef &S, const double *pose_init7) {
         unsigned char *mask = nullptr;
         cudaStream_t main_stream = c->stream;
         if (fork_gf && t == 0) c->stream = c->stream3;
-        rc = gf_select_set_device(c, t, sets[t], d_pose, sinfo, P.gf_method, (double)P.gf_ratio,
+        rc = gf_select_set_device(c, t, sets[t], d_pose, solve.sqrt_info, P.gf_method, (double)P.gf_ratio,
                                   (unsigned long long)P.gf_seed + 2ull * (unsigned long long)outer + (unsigned long long)t, &mask);
         c->stream = main_stream;
         if (rc) return rc;
@@ -94,17 +90,14 @@ int scan2map_enqueue(Ctx *c, const ScanRef &S, const double *pose_init7) {
     // :537-582 residual blocks + Evaluate -> J^T J -> evalDegenracy, and iteration 0 of ceres::Solve.  The device
     // only needs the degeneracy decision; scan2map_finish fills in the eigenvalue report of the last iteration.
     if (P.gf_method != 0) stamp(c, "gf");
-    c->want_eig = 0;
-    c->lin_two_pass = c->fuse_iter && P.max_inner == 1;  // the one LM iteration's second evaluation rides in the same launch
-    rc = linearize_device(c, sets, 2, sinfo, P.huber_a, nullptr, 1, 1, nullptr);
-    c->want_eig = 1;
-    const bool second_done = c->lin_two_pass;
-    c->lin_two_pass = false;
+    // max_inner == 1: the candidate of the one LM iteration is evaluated in the same launch
+    bool second_done = false;
+    rc = linearize_device(c, sets, 2, solve, kEvalBegin, nullptr, nullptr, defer, c->fuse_iter && P.max_inner == 1, &second_done);
     if (rc) return rc;
     stamp(c, second_done ? "linearize x2" : "linearize");
     // :586-596 ceres::Solve, at most max_inner LM iterations; the device raises `done`
     for (int it = 0; it < P.max_inner && !second_done; it++) {
-      rc = linearize_device(c, sets, 2, sinfo, P.huber_a, nullptr, 2, 2, nullptr);
+      rc = linearize_device(c, sets, 2, solve, kEvalCandidate);
       if (rc) return rc;
       stamp(c, "linearize (candidate)");
       if (P.max_inner > 1) {
@@ -166,8 +159,7 @@ int scan2map_finish(Ctx *c, const ScanRef &S, const double *pose_init7, double *
     // evalDegenracy's eigenvalues (lidar_mapper_keyframe.cpp:1172-1204): the device decides degeneracy with a
     // Cholesky test of H - thre*I and only runs the eigen-solver when that fails; the report of a healthy Solve is
     // computed here from the same H.
-    const double thre = c->lm_eig_thre >= 0.0 ? c->lm_eig_thre : c->params.eig_thre;
-    if (!hs->is_degenerate && !hs->skipped && hs->rows > 0 && thre > 0.0) eig_report_host(hs->H0, stats->eig);
+    if (!hs->is_degenerate && !hs->skipped && hs->rows > 0 && c->params.eig_thre > 0.0) eig_report_host(hs->H0, stats->eig);
     stats->n_surf_in = h_cnt[0], stats->n_corner_in = h_cnt[1];
   }
   return MLOAM_OK;

@@ -35,13 +35,10 @@ struct LinArgs {
   FeatSetDev set[2];
   int n_sets;
   double sqrt_info, huber_a;
-  const double *pose;      // explicit pose (7 doubles) or null
-  const LMState *state;    // state->x (use_state 1) / state->xc (use_state 2)
-  int use_state;
-  int respect_done;
+  const double *pose;      // where pass 0 evaluates: an explicit pose, LMState::x or LMState::xc (7 doubles)
+  const int *done;         // candidate evaluation: LMState::done (a terminated Solve has nothing to evaluate), else null
   // fused LM tail (single GPU): the block that finishes last reduces the partials and advances the state machine
   int lm_mode;             // 1 | 2, or 0: no tail (partials only)
-  int want_eig;
   double eig_thre;
   unsigned *ticket;        // zero between launches
   LMState *state_rw;
@@ -56,7 +53,7 @@ struct LinArgs {
   int fit_check_fov;
 };
 
-__device__ __noinline__ void lm_tail(const double *partials, int n_blocks, LMState *gst, int mode, double eig_thre, int want_eig, double *out_ne,
+__device__ __noinline__ void lm_tail(const double *partials, int n_blocks, LMState *gst, int mode, double eig_thre, double *out_ne,
                                      const P2PView *p2p);
 
 template <int KFIT>
@@ -64,19 +61,15 @@ __global__ void __launch_bounds__(LIN_THREADS) k_linearize(LinArgs a, double *__
   __shared__ double sm[LIN_THREADS / 32][NE_PACK];
   __shared__ bool is_last;
   __shared__ int barrier_failed;
-  if (a.respect_done && a.state && a.state->done) {  // Solve already terminated: nothing to evaluate
-    if (a.lm_mode != 0 && blockIdx.x == 0 && threadIdx.x == 0) a.state_rw->work[0] = 0, a.state_rw->work[1] = 0;
-    return;
-  }
+  if (a.done && *a.done) return;  // Solve already terminated: nothing to evaluate
   volatile unsigned *const gen = a.ticket + 1;
   const unsigned gen0 = a.two_pass ? *gen : 0u;  // read before this block's ticket: the release cannot have happened yet
 #pragma unroll 1
   for (int pass = 0; pass < (a.two_pass ? 2 : 1); pass++) {
   double xs[7];
   if (pass == 0) {
-    const double *px = a.use_state == 1 ? a.state->x : (a.use_state == 2 ? a.state->xc : a.pose);
 #pragma unroll
-    for (int k = 0; k < 7; k++) xs[k] = px[k];
+    for (int k = 0; k < 7; k++) xs[k] = a.pose[k];
   } else {
     // grid barrier: the block that ran the tail of pass 0 publishes the state and bumps the generation word
     if (threadIdx.x == 0) {
@@ -212,7 +205,7 @@ __global__ void __launch_bounds__(LIN_THREADS) k_linearize(LinArgs a, double *__
     return;
   }
   __threadfence();
-  lm_tail(partials, (int)gridDim.x, a.state_rw, pass == 0 ? a.lm_mode : 2, a.eig_thre, pass == 0 ? a.want_eig : 1, nullptr, a.p2p);
+  lm_tail(partials, (int)gridDim.x, a.state_rw, pass == 0 ? a.lm_mode : 2, a.eig_thre, nullptr, a.p2p);
   __threadfence();  // the state (written by all threads of this block) before the ticket reset and the release
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -421,7 +414,7 @@ __device__ void unpack_ne(const double *ne, double *H, double *g) {
 
 // One thread advances the state machine on a shared-memory copy of the state (lm_tail stages it in and out).
 // mode 1: begin a Solve with the evaluation at x.  mode 2: digest the evaluation at xc.
-__device__ void lm_advance(LMState *st, const double *ne, int mode, double eig_thre, int want_eig) {
+__device__ void lm_advance(LMState *st, const double *ne, int mode, double eig_thre) {
   double H[36], g[6];
   unpack_ne(ne, H, g);
   const double cost = ne[NE_H + NE_G];
@@ -444,10 +437,9 @@ __device__ void lm_advance(LMState *st, const double *ne, int mode, double eig_t
     st->is_degenerate = 0;
     for (int i = 0; i < 6; i++) st->eig[i] = 0.0;
     // lambda_min(H) > eig_thre  <=>  H - eig_thre*I is positive definite: one 6x6 Cholesky decides the common,
-    // non-degenerate case; the Jacobi eigen-solver only runs when a direction is (nearly) degenerate or when the
-    // caller asked for the eigenvalue report (want_eig: last outer iteration).
+    // non-degenerate case; the Jacobi eigen-solver only runs when a direction is (nearly) degenerate.
     bool need_eig = st->rows > 0 && eig_thre > 0.0;
-    if (need_eig && !want_eig) {
+    if (need_eig) {
       double S[36];
       for (int i = 0; i < 36; i++) S[i] = H[i] - ((i % 7 == 0) ? eig_thre : 0.0);
       double inv_diag[6];
@@ -474,6 +466,9 @@ __device__ void lm_advance(LMState *st, const double *ne, int mode, double eig_t
             st->V_update[i * 6 + j] = s;
           }
     }
+    // Compiler barrier: the state is re-read from shared memory below instead of being held in registers across the
+    // degeneracy test (which would add spills to lm_tail and stack to every kernel that calls it).
+    asm volatile("" ::: "memory");
     double xn = 0;
     for (int k = 0; k < 7; k++) xn += st->x[k] * st->x[k];
     st->x_norm = sqrt(xn);
@@ -538,7 +533,7 @@ __device__ void lm_advance(LMState *st, const double *ne, int mode, double eig_t
 // flags carry this exchange's epoch, and adds the slots in rank order — the same order on every rank, so all ranks
 // advance bit-identical states.  Slots and flags are double-buffered by the parity of the epoch: a rank can only be
 // one exchange ahead of the slowest one, so a slot is never overwritten before it has been read.
-__device__ __noinline__ void lm_tail(const double *partials, int n_blocks, LMState *gst, int mode, double eig_thre, int want_eig, double *out_ne,
+__device__ __noinline__ void lm_tail(const double *partials, int n_blocks, LMState *gst, int mode, double eig_thre, double *out_ne,
                                      const P2PView *p2p) {
   __shared__ double ne[NE_PACK];
   __shared__ unsigned long long p2p_epoch;
@@ -620,9 +615,8 @@ __device__ __noinline__ void lm_tail(const double *partials, int n_blocks, LMSta
     __syncthreads();
   }
   if (threadIdx.x == 0) {
-    s.work[0] = 0, s.work[1] = 0;  // re-arm the match work queues
     const long long t1 = clock64();
-    lm_advance(&s, ne, mode, eig_thre, want_eig);
+    lm_advance(&s, ne, mode, eig_thre);
     if (p2p && p2p_timeout) s.done = 1, s.termination = 9;  // exchange failed: the state is not trustworthy
     s.dbg_cycles[0] += t1 - t0, s.dbg_cycles[1] += clock64() - t1, s.dbg_cycles[2] += 1;
   }
@@ -635,8 +629,8 @@ __device__ __noinline__ void lm_tail(const double *partials, int n_blocks, LMSta
 }
 
 __global__ void __launch_bounds__(LM_THREADS) k_lm(const double *__restrict__ partials, int n_blocks, LMState *st, int mode, double eig_thre,
-                                                  int want_eig, double *__restrict__ out_ne) {
-  lm_tail(partials, n_blocks, st, mode, eig_thre, want_eig, out_ne, nullptr);
+                                                  double *__restrict__ out_ne) {
+  lm_tail(partials, n_blocks, st, mode, eig_thre, out_ne, nullptr);
 }
 
 __global__ void k_lm_init(LMState *st, const double *pose7, int max_inner, int min_corr) {
@@ -646,7 +640,6 @@ __global__ void k_lm_init(LMState *st, const double *pose7, int max_inner, int m
     st->min_corr = min_corr, st->skipped = 0;
     st->done = 0, st->termination = 0, st->total_iterations = 0, st->iteration = 0;
     st->is_degenerate = 0, st->rows = 0, st->n_valid[0] = st->n_valid[1] = 0;
-    st->work[0] = st->work[1] = 0;
     st->cost = 0, st->initial_cost = 0;
     for (int i = 0; i < 36; i++) st->V_update[i] = (i % 7 == 0) ? 1.0 : 0.0, st->H0[i] = 0, st->H[i] = 0;
     for (int i = 0; i < 6; i++) st->eig[i] = 0, st->g[i] = 0;
@@ -654,22 +647,21 @@ __global__ void k_lm_init(LMState *st, const double *pose7, int max_inner, int m
   }
 }
 
-int lm_init_state(Ctx *c, const double *pose7_host, int max_inner, double eig_thre) {
-  (void)eig_thre;
+int lm_init_state(Ctx *c, const double *pose7_host, int max_inner, int min_corr) {
   MLOAM_CUDA_OK(c, c->lm_state.reserve(sizeof(LMState) + 64));
   // stage the pose through pinned memory so the copy is truly asynchronous
   double *stage = reinterpret_cast<double *>(c->pinned);
   for (int k = 0; k < 7; k++) stage[k] = pose7_host[k];
   double *d_stage = c->scratch[7].as<double>();
   MLOAM_CUDA_OK(c, cudaMemcpyAsync(d_stage, stage, 7 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-  k_lm_init<<<1, 32, 0, c->stream>>>(c->lm_state.as<LMState>(), d_stage, max_inner, c->lm_min_corr);
+  k_lm_init<<<1, 32, 0, c->stream>>>(c->lm_state.as<LMState>(), d_stage, max_inner, min_corr);
   c->launches++;
   MLOAM_CUDA_OK(c, cudaGetLastError());
   return MLOAM_OK;
 }
 
-int linearize_device(Ctx *c, const FeatSet *sets, int n_sets, double sqrt_info, double huber_a, const double *d_pose7,
-                     int use_state, int lm_mode, double *d_out30) {
+int linearize_device(Ctx *c, const FeatSet *sets, int n_sets, const SolveCfg &cfg, LinEval eval, const double *d_pose7,
+                     double *d_out30, const PendingFit *fit, bool two_pass, bool *two_pass_done) {
   LinArgs a;
   int n_total = 0;
   for (int s = 0; s < 2; s++) {
@@ -683,11 +675,10 @@ int linearize_device(Ctx *c, const FeatSet *sets, int n_sets, double sqrt_info, 
       a.set[s].sinfo = nullptr, a.set[s].mask = nullptr;
     }
   }
-  const int want_eig = c->want_eig;
-  a.n_sets = n_sets, a.sqrt_info = sqrt_info, a.huber_a = huber_a, a.pose = d_pose7;
-  a.state = c->lm_state.as<LMState>();
-  a.use_state = use_state;
-  a.respect_done = (lm_mode == 2) ? 1 : 0;
+  LMState *st = c->lm_state.as<LMState>();
+  a.n_sets = n_sets, a.sqrt_info = cfg.sqrt_info, a.huber_a = cfg.huber_a;
+  a.pose = eval == kEvalBegin ? st->x : (eval == kEvalCandidate ? st->xc : d_pose7);
+  a.done = eval == kEvalCandidate ? &st->done : nullptr;
   int nb = (n_total + LIN_THREADS - 1) / LIN_THREADS;
   if (nb < 1) nb = 1;
   // n_total is a launch upper bound (device-side counts are usually far smaller): 64 blocks x 256 threads cover a
@@ -701,31 +692,23 @@ int linearize_device(Ctx *c, const FeatSet *sets, int n_sets, double sqrt_info, 
     MLOAM_CUDA_OK(c, cudaMemsetAsync(ticket, 0, sizeof(double), c->stream));
     c->ticket_zeroed_for = c->partials.p;
   }
-  const double eig_thre = c->lm_eig_thre >= 0.0 ? c->lm_eig_thre : c->params.eig_thre;
-  const bool collective = c->nccl_comm && c->p2p_collective;  // sum over the ranks wanted for this solve
-  const bool fused = lm_mode != 0 && (!collective || c->p2p_on) && !d_out30;
+  const bool collective = c->nccl_comm && cfg.collective;  // sum over the ranks wanted for this solve
+  const bool fused = eval != kEvalAtPose && (!collective || c->p2p_on) && !d_out30;
   // only the collective solves (scan2map on every rank in lock-step) exchange; per-rank solves on the same context — the tracker,
-  // mloam_normal_equations — stay local (c->p2p_collective is raised by scan2map_enqueue alone)
-  a.p2p = (fused && c->p2p_on && c->p2p_collective) ? static_cast<const P2PView *>(c->p2p_view) : nullptr;
-  a.lm_mode = fused ? lm_mode : 0, a.want_eig = want_eig, a.eig_thre = eig_thre, a.ticket = ticket;
-  a.state_rw = c->lm_state.as<LMState>();
+  // mloam_normal_equations — stay local
+  a.p2p = (fused && c->p2p_on && cfg.collective) ? static_cast<const P2PView *>(c->p2p_view) : nullptr;
+  a.lm_mode = fused ? eval : 0, a.eig_thre = cfg.eig_thre, a.ticket = ticket;
+  a.state_rw = st;
   // both evaluations of an LM iteration in one launch: only with the fused tail (the barrier is released by the block that ran it)
-  a.two_pass = (c->lin_two_pass && fused && lm_mode == 1) ? 1 : 0;
-  c->lin_two_pass = a.two_pass != 0;
+  a.two_pass = (two_pass && fused && eval == kEvalBegin) ? 1 : 0;
+  if (two_pass_done) *two_pass_done = a.two_pass != 0;
   // a fit the matcher deferred to this evaluation
-  int kfit = 0;
+  const int kfit = fit ? fit->K : 0;
   memset(a.fit, 0, sizeof(a.fit));
   a.fit_min_plane_dis = 0.f, a.fit_check_fov = 0;
-  if (c->pending_fit.K) {
-    if (lm_mode != 1 || n_sets != 2 || (c->pending_fit.K != 5 && c->pending_fit.K != 10)) {
-      c->err = "linearize: a deferred fit is pending but this is not the first evaluation of a solve";
-      c->pending_fit.K = 0;
-      return MLOAM_E_STATE;
-    }
-    kfit = c->pending_fit.K;
-    a.fit[0] = c->pending_fit.set[0], a.fit[1] = c->pending_fit.set[1];
-    a.fit_min_plane_dis = c->pending_fit.min_plane_dis, a.fit_check_fov = c->pending_fit.check_fov;
-    c->pending_fit.K = 0;
+  if (kfit) {
+    a.fit[0] = fit->set[0], a.fit[1] = fit->set[1];
+    a.fit_min_plane_dis = fit->min_plane_dis, a.fit_check_fov = fit->check_fov;
   }
   {
     ProfScope ps(c, "linearize");
@@ -738,23 +721,22 @@ int linearize_device(Ctx *c, const FeatSet *sets, int n_sets, double sqrt_info, 
     MLOAM_CUDA_OK(c, cudaGetLastError());
     return MLOAM_OK;
   }
-  if (collective && lm_mode != 0) {
+  if (collective && eval != kEvalAtPose) {
     // multi-GPU: rank-local sum -> NCCL all-reduce of the 30 packed doubles -> identical LM step on every rank
     double *ne = c->partials.as<double>() + (size_t)NE_PACK * max_nb;
     {
       ProfScope ps(c, "lm");
-      k_lm<<<1, LM_THREADS, 0, c->stream>>>(c->partials.as<double>(), nb, c->lm_state.as<LMState>(), 0, 0.0, 0, ne);
+      k_lm<<<1, LM_THREADS, 0, c->stream>>>(c->partials.as<double>(), nb, st, 0, 0.0, ne);
       c->launches++;
     }
     int rc = comm_allreduce_doubles(c, ne, NE_PACK);
     if (rc) return rc;
     ProfScope ps(c, "lm");
-    k_lm<<<1, LM_THREADS, 0, c->stream>>>(ne, 1, c->lm_state.as<LMState>(), lm_mode, (c->lm_eig_thre >= 0.0 ? c->lm_eig_thre : c->params.eig_thre), want_eig, d_out30);
+    k_lm<<<1, LM_THREADS, 0, c->stream>>>(ne, 1, st, eval, cfg.eig_thre, d_out30);
     c->launches++;
   } else {
     ProfScope ps(c, "lm");
-    k_lm<<<1, LM_THREADS, 0, c->stream>>>(c->partials.as<double>(), nb, c->lm_state.as<LMState>(), lm_mode, (c->lm_eig_thre >= 0.0 ? c->lm_eig_thre : c->params.eig_thre), want_eig,
-                                  d_out30);
+    k_lm<<<1, LM_THREADS, 0, c->stream>>>(c->partials.as<double>(), nb, st, eval, cfg.eig_thre, d_out30);
     c->launches++;
   }
   MLOAM_CUDA_OK(c, cudaGetLastError());

@@ -164,18 +164,9 @@ int track_cloud_device(Ctx *c, const float4 *d_prev_less_sharp, int n_pls, const
   rc = reserve_feat(c, 1, n_cf);
   if (rc) return rc;
   const int max_outer = 2, max_inner = 4;  // :44, :114
-  const double huber_a = 0.1;              // :47
-  // per-solve settings travel through context fields that lm_init_state / linearize_device read: restored on every exit path
-  struct SolveSettings {
-    Ctx *c;
-    explicit SolveSettings(Ctx *cc) : c(cc) {
-      c->lm_min_corr = 10;  // :64-68
-      c->lm_eig_thre = 0.0; // evalDegenracy is commented out in trackCloud (:101-108)
-    }
-    ~SolveSettings() { c->lm_min_corr = 0, c->lm_eig_thre = -1.0, c->want_eig = 1; }
-  } settings(c);
-  rc = lm_init_state(c, pose_ini7, max_inner, 0.0);
-  c->lm_min_corr = 0;
+  // Huber 0.1 (:47); evalDegenracy is commented out in trackCloud (:101-108)
+  const SolveCfg cfg{1.0, 0.1, 0.0, false};
+  rc = lm_init_state(c, pose_ini7, max_inner, 10);  // :64-68
   if (rc) return rc;
   LMState *st = c->lm_state.as<LMState>();
   int *h_done = reinterpret_cast<int *>(reinterpret_cast<char *>(c->pinned) + 2048);
@@ -188,12 +179,10 @@ int track_cloud_device(Ctx *c, const float4 *d_prev_less_sharp, int n_pls, const
     rc = match_from_scan_device(c, MLOAM_MAP_SCAN_SURF, 's', d_cur_flat, n_cf, st->x, c->feat_valid[1].as<unsigned char>(),
                                 c->feat_coeff[1].as<float>(), nullptr);
     if (rc) break;
-    c->want_eig = 0;
-    rc = linearize_device(c, sets, 2, 1.0, huber_a, nullptr, 1, 1, nullptr);
-    c->want_eig = 1;
+    rc = linearize_device(c, sets, 2, cfg, kEvalBegin);
     if (rc) break;
     for (int it = 0; it < max_inner; it++) {
-      rc = linearize_device(c, sets, 2, 1.0, huber_a, nullptr, 2, 2, nullptr);
+      rc = linearize_device(c, sets, 2, cfg, kEvalCandidate);
       if (rc) break;
       if (cudaMemcpyAsync(h_done, &st->done, sizeof(int), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
           cudaStreamSynchronize(c->stream) != cudaSuccess) {
@@ -204,7 +193,6 @@ int track_cloud_device(Ctx *c, const float4 *d_prev_less_sharp, int n_pls, const
       if (*h_done) break;
     }
   }
-  c->lm_eig_thre = -1.0;
   if (rc) return rc;
   LMState *hs = reinterpret_cast<LMState *>(reinterpret_cast<char *>(c->pinned) + 4096);
   MLOAM_CUDA_OK(c, cudaMemcpyAsync(hs, st, sizeof(LMState), cudaMemcpyDeviceToHost, c->stream));

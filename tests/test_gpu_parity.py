@@ -811,10 +811,13 @@ def test_frame_lookahead_is_exact(mloam, n_lidars, gf):
 
 
 @pytest.mark.parametrize("outer,inner,guess", [(6, 1, 0.0), (3, 4, 0.0), (4, 1, 0.6)])
-def test_seeded_reassociation_is_exact(mloam, c1, outer, inner, guess):
+@pytest.mark.parametrize("switch,off,on", [("MLOAM_DISABLE_SEEDS", "1", "0"), ("MLOAM_FUSE_ITER", "0", "1")], ids=["seeds", "fuse_iter"])
+def test_seeded_reassociation_is_exact(mloam, c1, switch, off, on, outer, inner, guess):
     """From the second re-association on, the kNN is seeded with the previous neighbour lists and unchanged lists keep
     their fit.  That is an exact shortcut: poses, match counts and the Hessian must be BIT-identical to the blind
-    search — also when the pose moves a lot between iterations (a poor initial guess)."""
+    search — also when the pose moves a lot between iterations (a poor initial guess).  The same holds for the fused
+    evaluation (fit inside the first evaluation, both evaluations of an LM iteration in one launch) against one launch
+    per step."""
     import os
 
     p = mloam.default_params()
@@ -822,12 +825,12 @@ def test_seeded_reassociation_is_exact(mloam, c1, outer, inner, guess):
     init = np.array(c1["init"], dtype=np.float64)
     init[:3] += guess
     res = []
-    for disable in ("1", "0"):
-        os.environ["MLOAM_DISABLE_SEEDS"] = disable
+    for value in (off, on):
+        os.environ[switch] = value
         try:
             cx = mloam.Context(0, p)
         finally:
-            os.environ.pop("MLOAM_DISABLE_SEEDS")
+            os.environ.pop(switch)
         cx.map_build(1, c1["surf_map"], 0.5)
         cx.map_build(0, c1["corner_map"], 0.5)
         res.append(cx.scan2map(c1["surf_scan"], c1["corner_scan"], init))
